@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- candidate-fits/sec of the cross-validated grid search (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...      (N > 1)
 
 A "step" is one pass of the hot path over the whole workload: every (candidate, fold) fit+score task of
@@ -207,6 +207,14 @@ def parity_block(w, test_scores):
             "max_abs_diff_mean_test_score": dm, "split_scores_equal": bool(np.array_equal(test_scores, g["test_scores"]))}
 
 
+def dump_outputs(path, key, m):
+    """The split scores the last timed step returned ([candidates][splits] float64) as <path>/<key>_{test,train}_scores.npy.
+    fit_time / score_time, the other arrays of that step, are wall-clock timings and would differ on every run."""
+    os.makedirs(path, exist_ok=True)
+    for part in ("test", "train"):
+        np.save(os.path.join(path, "%s_%s_scores.npy" % (key, part)), np.asarray(m[part], np.float64))
+
+
 def tf32_peak_tflops():
     """cuBLAS TF32 GEMM throughput on this GPU (the denominator for the tcgen05 kind::tf32 contraction kernel)."""
     import torch
@@ -310,11 +318,11 @@ class Runner:
         r = dict(zip(keys_max + ["wall", "e2e_wall"], [float(x) for x in tm.cpu()]))
         r.update(zip(keys_sum, [float(x) for x in ts.cpu()]))
         r["phase_mean"] = dict(zip(keys_max, [float(x) / max(self.world, 1) for x in tavg.cpu()]))
-        r.update(test=out["test"], e2e_prof=e2e_prof, clocks=clocks, steps=steps)
+        r.update(test=out["test"], train=out["train"], e2e_prof=e2e_prof, clocks=clocks, steps=steps)
         return r
 
 
-def secondary_entry(key, rank, world, local_rank, dist, steps, peaks):
+def secondary_entry(key, rank, world, local_rank, dist, steps, peaks, dump_dir=None):
     """One BASELINE config, strong-scaled over the ranks: value, e2e, parity vs golden, roofline of its dominant kernel."""
     from spark_sklearn_b200 import workloads as WL
     w = WL.make_workload(key)
@@ -323,6 +331,8 @@ def secondary_entry(key, rank, world, local_rank, dist, steps, peaks):
     m = run.measure(steps, 2)
     if rank != 0:
         return None
+    if dump_dir:
+        dump_outputs(dump_dir, key, m)
     fits, K = run.fits, steps
     ent = {"workload": "%s: %s(%s), %dx%d, %d candidates x cv=%d = %d fits" % (
                w["name"], "GridSearchCV" if w["search"] == "grid" else "RandomizedSearchCV", w["estimator"],
@@ -359,7 +369,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the split scores of every measured workload's last step to "
+                         "DIR/<workload>_{test,train}_scores.npy (float64; the inputs are seeded, so runs and builds compare)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     # stdout carries exactly ONE line (the JSON): libraries that print there (NCCL's version banner, joblib) go to stderr
     sys.stdout.flush()
     real_stdout = os.fdopen(os.dup(1), "w")
@@ -416,6 +433,8 @@ def main():
     m = run.measure(a.steps, W_, sampler)
     test_scores = m["test"]
     fits = run.fits
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, a.workload, m)
 
     peak, peak_src = measured_peaks()
     secondary = None
@@ -423,7 +442,7 @@ def main():
         tf32 = tf32_peak_tflops() if rank == 0 else 0.0
         secondary = {}
         for key in ("c4", "c3", "c5"):
-            ent = secondary_entry(key, rank, world, local_rank, dist, min(max(a.steps, 1), 5), (peak, tf32))
+            ent = secondary_entry(key, rank, world, local_rank, dist, a.steps, (peak, tf32), a.dump_outputs)
             if rank == 0:
                 secondary[key] = ent
         if rank == 0:
