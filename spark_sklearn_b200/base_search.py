@@ -140,7 +140,12 @@ class B200BaseSearchCV(BaseSearchCV):
             array_stds = np.sqrt(np.average((array - array_means[:, np.newaxis]) ** 2, axis=1, weights=weights))
             results['std_%s' % key_name] = array_stds
             if rank:
-                results["rank_%s" % key_name] = np.asarray(rankdata(-array_means, method='min'), dtype=np.int32)
+                # a NaN mean (a split scored error_score=nan) ranks last, as in scikit-learn; all NaN: all rank 1
+                if np.isnan(array_means).all():
+                    ranked = np.ones_like(array_means)
+                else:
+                    ranked = rankdata(-np.nan_to_num(array_means, nan=np.nanmin(array_means) - 1), method='min')
+                results["rank_%s" % key_name] = np.asarray(ranked, dtype=np.int32)
 
         _store('test_score', test_scores, splits=True, rank=True,
                weights=test_sample_counts if self.iid else None)

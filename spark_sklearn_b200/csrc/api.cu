@@ -17,6 +17,8 @@ static std::string g_create_error;
 // scikit-learn's count-based scores (metrics/_classification.py) from cnt[class][3] = {support, tp, predicted}, float64.
 // Undefined ratios follow zero_division="warn": 0.0.  accuracy_score :187; balanced_accuracy_score :2362 (mean recall over
 // the classes present in y_true); precision_recall_fscore_support :1573 with beta = 1: f = 2 tp / (2 tp + fp + fn).
+// The averages run over the labels present in y_true or y_pred: a class with support + predicted == 0 adds nothing to the
+// weighted f1 (weight 0) or to balanced accuracy (only y_true's classes), and is left out of the macro mean.
 double gs_score_from_counts(int kind, int pos_class, int n_classes, const int *cnt)
 {
     auto sup = [&](int c) { return (double)cnt[c * 3 + 0]; };
@@ -37,9 +39,11 @@ double gs_score_from_counts(int kind, int pos_class, int n_classes, const int *c
     case GS_SCORE_PRECISION: return prd(pos_class) > 0 ? tp(pos_class) / prd(pos_class) : 0.0;
     case GS_SCORE_RECALL: return sup(pos_class) > 0 ? tp(pos_class) / sup(pos_class) : 0.0;
     case GS_SCORE_F1_MACRO: {
-        double s = 0;
-        for (int c = 0; c < n_classes; c++) s += f1c(c);
-        return s / n_classes;
+        // mean over the labels of y_true and y_pred (unique_labels, :1573): a class of the dataset that is neither in this
+        // set nor predicted for it does not count
+        double s = 0; int k = 0;
+        for (int c = 0; c < n_classes; c++) if (sup(c) + prd(c) > 0) { s += f1c(c); k++; }
+        return s / k;                                                    // k >= 1: n > 0 rows were predicted
     }
     case GS_SCORE_F1_MICRO: return correct / n;                         // single-label: micro f1 == accuracy
     case GS_SCORE_F1_WEIGHTED: {
@@ -287,10 +291,11 @@ int gs_set_data(gs_handle *h, const void *X, int32_t x_dtype, int64_t n, int64_t
     GS_CUDA(cudaMemcpyAsync(h->dFold.p, h->fold.data(), (size_t)n, cudaMemcpyHostToDevice, h->stream));
     GS_CUDA(cudaMemcpyAsync(h->dTe.p, h->te_mask.data(), (size_t)n * 16, cudaMemcpyHostToDevice, h->stream));
     GS_CUDA(cudaMemcpyAsync(h->dTr.p, h->tr_mask.data(), (size_t)n * 16, cudaMemcpyHostToDevice, h->stream));
+    h->yt.clear();
     if (y_target) {
-        std::vector<float> yt(n);
-        for (int64_t i = 0; i < n; i++) yt[i] = y_target[h->perm[i]];
-        GS_CUDA(cudaMemcpyAsync(h->dYt.p, yt.data(), (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
+        h->yt.resize(n);
+        for (int64_t i = 0; i < n; i++) h->yt[i] = y_target[h->perm[i]];
+        GS_CUDA(cudaMemcpyAsync(h->dYt.p, h->yt.data(), (size_t)n * 4, cudaMemcpyHostToDevice, h->stream));
         GS_CUDA(cudaStreamSynchronize(h->stream));
     }
     cudaEventRecord(e1, h->stream);

@@ -98,6 +98,7 @@ struct gs_handle {
     bool classification = false;
     std::vector<int32_t> perm;        // internal row -> original row
     std::vector<int32_t> yc;          // [n] class ids, internal order
+    std::vector<float> yt;            // [n] regression targets, internal order (empty for a classification dataset)
     std::vector<int8_t> fold;         // [n] fold ids, internal order (partition splitters; Ridge's fold blocks)
     std::vector<uint64_t> te_mask, tr_mask;   // [n][2] split membership, internal order
     bool partition = true;            // the splits are a partition into test folds whose complements train (gs_set_data's fold ids)

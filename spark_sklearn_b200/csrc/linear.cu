@@ -751,12 +751,29 @@ int ridge_run(gs_handle *h, int n_cand, const double *alpha, int fit_intercept, 
         GS_CUDA(cudaMemcpyAsync(out.data(), dOut, out.size() * 8, cudaMemcpyDeviceToHost, st));
         cudaEventRecord(ev[3], st);
         GS_CUDA(cudaStreamSynchronize(st));
-        for (int g = 0; g < groups; g++)
+        // R^2 of a set whose targets are all equal: the total sum of squares is 0, and the one ridge_r2_kernel divides by is
+        // float32 rounding noise of the Gram statistics (a large finite value of either sign, or inf / NaN).  scikit-learn's
+        // r2_score (force_finite=True) gives 1.0 for an exact prediction and 0.0 otherwise; the residual from Gram statistics
+        // cannot certify an exact zero, so such a set scores 0.0.
+        auto constant_targets = [&](int k, bool test) {
+            bool any = false;
+            float v = 0.f;
+            for (int r = 0; r < n; r++) {
+                if (!(test ? h->is_test(r, k) : h->is_train(r, k))) continue;
+                if (!any) { v = h->yt[r]; any = true; }
+                else if (h->yt[r] != v) return false;
+            }
+            return any;
+        };
+        for (int g = 0; g < groups; g++) {
+            const bool r2 = h->score_kind == GS_SCORE_DEFAULT;
+            const bool const_te = r2 && constant_targets(g, true), const_tr = r2 && train_scores && constant_targets(g, false);
             for (int c = 0; c < n_cand; c++) {
                 const size_t s = (size_t)g * n_cand + c;
-                test_scores[(size_t)c * ns + g] = out[s * 2];
-                if (train_scores) train_scores[(size_t)c * ns + g] = out[s * 2 + 1];
+                test_scores[(size_t)c * ns + g] = const_te ? 0.0 : out[s * 2];
+                if (train_scores) train_scores[(size_t)c * ns + g] = const_tr ? 0.0 : out[s * 2 + 1];
             }
+        }
         h->prof.d2h_bytes = (int64_t)out.size() * 8;
     } else {
         std::vector<float> w(dp), shift(d + 1);
